@@ -459,6 +459,28 @@ def copy_ceiling(torch, up_bytes, down_bytes, seconds=0.6):
     return n / run(n)
 
 
+def dump_outputs(out_dir, outputs, budget_bytes=60 << 20):
+    """Writes what the timed path returned as out_dir/<name>.npy (float32, exact for these integer types).
+    outputs: {name: (device uint8 buffers, numpy dtype, elements per buffer)}; the buffers are concatenated in order.
+    An output larger than its share of the budget is written as a fixed sample: element indices drawn with a seeded
+    generator and sorted, so two runs with the same arguments sample the same elements."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    cap = budget_bytes // 4 // len(outputs)
+    for name, (bufs, dtype, n) in outputs.items():
+        dtype = np.dtype(dtype)
+        total = len(bufs) * n
+        idx = None if total <= cap else np.unique(np.random.default_rng(0).integers(0, total, cap))
+        parts = []
+        for i, buf in enumerate(bufs):
+            v = buf[:n * dtype.itemsize].view(torch.uint8 if dtype.itemsize == 1 else torch.int16)
+            if idx is not None:
+                sel = idx[(idx >= i * n) & (idx < (i + 1) * n)] - i * n
+                v = v[torch.from_numpy(sel).to(v.device)]
+            parts.append(v.cpu().numpy().view(dtype))
+        np.save(os.path.join(out_dir, name + ".npy"), np.concatenate(parts).astype(np.float32))
+
+
 def run_ours(args, rank, world, local_rank):
     import torch
     pkg = importlib.import_module("cineform-sdk_b200")        # raises if libcfhd_b200.so is missing
@@ -531,6 +553,13 @@ def run_ours(args, rank, world, local_rank):
     launches = launches_per_step * args.steps
     ms_per_step = total_ms / args.steps
     value = aggregate_fps(world, B * args.steps, total_ms / 1000.0)
+    if args.dump_outputs and rank == 0:
+        # the last timed step's results, before the per-level timing below overwrites the buffers
+        outputs = {"coefficients": (d_pyr, np.int16, lay.coded_bytes // 2)}
+        if decode:
+            out_dtype = {"YUYV": np.uint8, "RG48": np.uint16}.get(CFG["fmt"], np.int16)
+            outputs["decoded"] = (d_out, out_dtype, lay.frame_bytes // np.dtype(out_dtype).itemsize)
+        dump_outputs(args.dump_outputs, outputs)
 
     # ---- parity spot check of what was just timed (decoded frame vs input) ----
     roundtrip_psnr = None
@@ -711,7 +740,12 @@ def main():
     ap.add_argument("--ref-iters", type=int, default=6, help="frames per host thread (at the full thread count) in the CPU baseline")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="CUDA path only: write the last timed step's coefficients (and decoded frames) of rank 0 as "
+                         "DIR/<name>.npy, float32; outputs over the 64 MB budget are a fixed seeded sample")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the CUDA path; --impl reference has none")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

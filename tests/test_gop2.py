@@ -12,6 +12,7 @@ import pytest
 
 import oracle_lib as ol
 import parity_util as pu
+from ref_golden import Golden
 
 GOLDEN = sorted(glob.glob(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "gop2_*.npz")))
 needs_ref = pytest.mark.skipif(not ol.ref_available(), reason="oracle/_ref not built (reference absent)")
@@ -237,30 +238,28 @@ def test_cuda_gop2_single_call(path):
         assert pu.psnr(out[:, 0::2], src[:, 0::2]) > 45.0
 
 
-@needs_ref
 @pytest.mark.parametrize("quality", [1, 2, 3, 4, 5, 6, 4 | (1 << 17)])
 @pytest.mark.parametrize("interlaced", [False, True])
-def test_gop2_quant_schedule_matches_reference(quality, interlaced):
-    """cfb_gop2_quant_for_quality == the divisors / prescale the reference's encoder really used (quantize.c:3480)."""
+def test_gop2_quant_schedule_matches_reference(request, quality, interlaced):
+    """cfb_gop2_quant_for_quality == the divisors / prescale the reference's encoder really used (quantize.c:3480;
+    stored in tests/golden/ref_digests.json)."""
     pkg = importlib.import_module("cineform-sdk_b200")
     w, h = 256, 64
-    ref_lib = ol.load_ref()
-    fa, fb = pu.qbist_yuy2(ref_lib, w, h, 1), pu.qbist_yuy2(ref_lib, w, h, 2)
-    ref_lib.ref_set_interlaced(1 if interlaced else 0)
-    try:
-        _, quant, prescale = pu.ref_encode_gop2(ref_lib, fa, fb, w, h, quality)
-    finally:
-        ref_lib.ref_set_interlaced(0)
+    coded = lambda k, d: d[1:] if k in (0, 1, 4) else d            # LL of wavelets 0, 1, 4 is never coded
+
+    def want():
+        ref_lib = ol.load_ref()
+        fa, fb = pu.qbist_yuy2(ref_lib, w, h, 1), pu.qbist_yuy2(ref_lib, w, h, 2)
+        ref_lib.ref_set_interlaced(1 if interlaced else 0)
+        try:
+            _, quant, prescale = pu.ref_encode_gop2(ref_lib, fa, fb, w, h, quality)
+        finally:
+            ref_lib.ref_set_interlaced(0)
+        return [prescale[0][:6]] + [[coded(k, quant[c][k][:2 if k == 2 else 4]) for k in range(6)] for c in range(3)]
     q = pkg.gop2_quant_for_quality(pkg.FrameDesc(w, h, pkg.PIXEL_YUYV), quality, interlaced)
-    assert [int(v) for v in q.prescale] == prescale[0][:6]
-    for c in range(3):
-        for k in range(6):
-            nb = 2 if k == 2 else 4
-            got = [int(q.divisor[c][k][b]) for b in range(nb)]
-            want = quant[c][k][:nb]
-            if k in (0, 1, 4):
-                got, want = got[1:], want[1:]            # their LL is never coded
-            assert got == want, (c, k, got, want)
+    got = [[int(v) for v in q.prescale]] + [[coded(k, [int(q.divisor[c][k][b]) for b in range(2 if k == 2 else 4)])
+                                             for k in range(6)] for c in range(3)]
+    Golden(request).check_values(got, want, "prescale, divisors per channel and wavelet")
 
 
 @needs_ref

@@ -11,6 +11,7 @@ import pytest
 
 import oracle_lib as ol
 import parity_util as pu
+from ref_golden import Golden
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 needs_ref = pytest.mark.skipif(not ol.ref_available(), reason="oracle/_ref not built (reference absent)")
@@ -46,33 +47,36 @@ def test_known_answer_sample_size():
     assert abs(sample.size - 592268) < 2048
 
 
-@needs_ref
 @pytest.mark.parametrize("quality", [1, 2, 3, 4, 5, 6, 4 | (1 << 17), 4 | (3 << 17)])
-def test_quant_schedule_matches_reference(pkg, quality):
+def test_quant_schedule_matches_reference(pkg, request, quality):
+    """Divisors and prescale of the reference's EncodeSample (a Qbist frame; stored in tests/golden/ref_digests.json)."""
     w, h = 256, 64
-    ref_lib = ol.load_ref()
-    frame = pu.qbist_yuy2(ref_lib, w, h, 1)
-    _, div, prescale, _ = pu.ref_encode_frame(ref_lib, frame, w, h, pu.COLOR_FORMAT_YUYV, 0, 3, quality)
+
+    def want():
+        ref_lib = ol.load_ref()
+        frame = pu.qbist_yuy2(ref_lib, w, h, 1)
+        _, div, prescale, _ = pu.ref_encode_frame(ref_lib, frame, w, h, pu.COLOR_FORMAT_YUYV, 0, 3, quality)
+        return [div, prescale[0]]
     q = pkg.quant_for_quality(pkg.FrameDesc(w, h, pkg.PIXEL_YUYV), quality)
-    assert q.table(3) == div
-    assert list(q.prescale) == prescale[0]
+    Golden(request).check_values([q.table(3), list(q.prescale)], want, "divisors, prescale")
 
 
-@needs_ref
 @pytest.mark.parametrize("quality", [1, 2, 3, 4, 5, 6, 4 | (1 << 17)])
-def test_interlaced_quant_schedule_matches_reference(pkg, quality):
+def test_interlaced_quant_schedule_matches_reference(pkg, request, quality):
     """parameters.progressive = 0 (CFHD_ENCODING_FLAGS_YUV_INTERLACED): quantize.c:490-541 rescales level 1."""
     w, h = 256, 64
-    ref_lib = ol.load_ref()
-    frame = pu.qbist_yuy2(ref_lib, w, h, 1)
-    ref_lib.ref_set_interlaced(1)
-    try:
-        _, div, prescale, _ = pu.ref_encode_frame(ref_lib, frame, w, h, pu.COLOR_FORMAT_YUYV, 0, 3, quality)
-    finally:
-        ref_lib.ref_set_interlaced(0)
+
+    def want():
+        ref_lib = ol.load_ref()
+        frame = pu.qbist_yuy2(ref_lib, w, h, 1)
+        ref_lib.ref_set_interlaced(1)
+        try:
+            _, div, prescale, _ = pu.ref_encode_frame(ref_lib, frame, w, h, pu.COLOR_FORMAT_YUYV, 0, 3, quality)
+        finally:
+            ref_lib.ref_set_interlaced(0)
+        return [div, prescale[0]]
     q = pkg.quant_for_quality(pkg.FrameDesc(w, h, pkg.PIXEL_YUYV), quality, interlaced=True)
-    assert q.table(3) == div
-    assert list(q.prescale) == prescale[0]
+    Golden(request).check_values([q.table(3), list(q.prescale)], want, "divisors, prescale")
 
 
 @needs_ref

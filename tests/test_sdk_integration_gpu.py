@@ -12,7 +12,9 @@ pytestmark = pytest.mark.gpu
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BUILD = os.path.join(ROOT, "integration", "_build")
 have = all(os.path.exists(os.path.join(BUILD, f)) for f in ("sdk_roundtrip", "sdk_roundtrip_ref", "TestCFHD", "libCFHDCodec.so"))
-needs_build = pytest.mark.skipif(not have, reason="integration/_build not present (built where /root/reference exists)")
+needs_build = pytest.mark.skipif(not have, reason="integration/_build not built: the shim and the programs it serves compile "
+                                                  "against the reference's headers and objects, so build() makes them only "
+                                                  "where the reference sources are present")
 
 
 def shim_stats(stderr):

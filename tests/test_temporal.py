@@ -1,5 +1,6 @@
 """Two-frame GOP building block: temporal Haar between two int16 planes (Codec/temporal.c:498 FilterTemporal16s,
-:9402 InvertTemporalQuant16s).  CPU: oracle vs the reference functions themselves (oracle/_ref).  GPU: CUDA vs oracle."""
+:9402 InvertTemporalQuant16s).  CPU: oracle vs the reference functions themselves (oracle/_ref, or their results stored
+in tests/golden/ref_digests.json).  GPU: CUDA vs oracle."""
 import ctypes as C
 import importlib
 
@@ -7,8 +8,8 @@ import numpy as np
 import pytest
 
 import oracle_lib as ol
+from ref_golden import Golden
 
-needs_ref = pytest.mark.skipif(not ol.ref_available(), reason="oracle/_ref not built (reference absent)")
 SHAPES = [(16, 4), (48, 6), (80, 5), (96, 7), (1920, 8), (960, 540)]
 
 
@@ -32,15 +33,13 @@ def _run(lib, prefix, a, b):
     return out
 
 
-@needs_ref
 @pytest.mark.parametrize("shape", SHAPES)
 @pytest.mark.parametrize("kind", ["small", "full"])
-def test_oracle_temporal_matches_reference(shape, kind):
+def test_oracle_temporal_matches_reference(request, shape, kind):
     """Saturating SSE2 body, int scalar tail (width % 40) and the precision-8 half-tone quirk, full int16 range."""
     w, h = shape
     a, b = _planes(np.random.default_rng(w + h), w, h, kind)
-    for got, want in zip(_run(ol.load_oracle(), "orc_", a, b), _run(ol.load_ref(), "ref_", a, b)):
-        assert np.array_equal(got, want)
+    Golden(request).check(_run(ol.load_oracle(), "orc_", a, b), lambda: _run(ol.load_ref(), "ref_", a, b))
 
 
 def test_oracle_temporal_roundtrip():
