@@ -202,6 +202,12 @@ def layout_for(desc):
     return out
 
 
+def v210_pitch(width):
+    """Smallest pitch of a V210 output frame: whole 6-pixel groups of 16 bytes (the inverse writes exactly this much per
+    row).  The SDK's own V210 frames round the row up to 128 bytes, which the inverse accepts as well."""
+    return (width + 5) // 6 * 16
+
+
 def device_numa_node(device):
     return int(lib().cfb_device_numa_node(device))
 

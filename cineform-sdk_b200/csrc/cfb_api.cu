@@ -62,6 +62,8 @@ cudaError_t stream_wait(cfb_context *ctx)
 
 static inline int align16(int x) { return (x + 15) & ~15; }
 static inline int64_t align64(int64_t x) { return (x + 63) & ~(int64_t)63; }
+// bytes of one V210 row: whole groups of 6 pixels in 4 32-bit words
+static inline int v210_row_bytes(int w) { return (w + 5) / 6 * 16; }
 
 static int channels_of(int fmt) { return fmt == CFB_PIXEL_BYR4 ? 4 : 3; }
 
@@ -825,6 +827,13 @@ cfb_error cfb_inverse_device(cfb_codec *cd, int n, void *const *d_pyramids, cons
         if (frame_pitch < out_w * bpp || (frame_pitch & 15)) { set_error("bad output pitch %d", frame_pitch); return CFB_ERROR_INVALID_ARGUMENT; }
         for (int c = 0; c < L.num_channels; c++)
             if (L.band[c][0][0].width < 16) { set_error("16-bit packed output needs level-1 bands at least 16 coefficients wide"); return CFB_ERROR_UNSUPPORTED; }
+    } else if (out_format == CFB_PIXEL_V210) {
+        // 10-bit packed 4:2:2: the YU64 rows >> 6 (decoder.c:26292 -> convert.c:13526 ConvertPlanarYUVToV210).  The reference
+        // renders V210 from a field transform only through its active-metadata path (decoder.c:26413), and reduced
+        // resolutions through ConvertLowpass16s10bitToV210 (decoder.c:23054): neither is built here
+        if (!is422) { set_error("V210 output needs a 4:2:2 codec"); return CFB_ERROR_BADFORMAT; }
+        if (cd->decode_res != CFB_RESOLUTION_FULL || cd->interlaced) { set_error("V210 output: full-resolution progressive decode only"); return CFB_ERROR_UNSUPPORTED; }
+        if (frame_pitch < v210_row_bytes(out_w) || (frame_pitch & 15)) { set_error("bad output pitch %d", frame_pitch); return CFB_ERROR_INVALID_ARGUMENT; }
     } else if (out_format >= CFB_PIXEL_RG30 && out_format <= CFB_PIXEL_DPX0) {
         // 10-bit packed RGB of an RGB 4:4:4 sample (decoder.c:26893 -> InvertHorizontalStrip16s.c:14812 ...RGB2RG30)
         if (!is444 || L.num_channels != 3 || L.precision != 12) { set_error("10-bit RGB output needs a three-channel 12-bit 4:4:4 codec"); return CFB_ERROR_BADFORMAT; }
@@ -954,9 +963,11 @@ cfb_error cfb_inverse_device(cfb_codec *cd, int n, void *const *d_pyramids, cons
                 p.tail_col[c] = (w - (w % 8) - 16) + 7;
             }
             if (out_format == CFB_PIXEL_RG48) CFB_CUDA(launch_inv_444_rg48(p, 0, ctx->stream));
-            else CFB_CUDA(launch_inv_422(p, true, ctx->stream));
+            else CFB_CUDA(launch_inv_422(p, kInv422OutYU64, ctx->stream));
+        } else if (out_format == CFB_PIXEL_V210) {
+            CFB_CUDA(launch_inv_422(p, kInv422OutV210, ctx->stream));
         } else {
-            CFB_CUDA(launch_inv_422(p, false, ctx->stream));
+            CFB_CUDA(launch_inv_422(p, kInv422Out8, ctx->stream));
         }
     }
     ctx->kernel_launches++;
@@ -990,8 +1001,11 @@ static cfb_error inv_output_geometry(const cfb_codec *cd, int out_format, int *r
     const int kk = cd->decode_res - 1;          // lowest level that is inverted (0 = all three)
     const bool rgb30 = (out_format >= CFB_PIXEL_RG30 && out_format <= CFB_PIXEL_DPX0);
     const int bpp = (out_format == CFB_PIXEL_YU64 || rgb30) ? 4 : (out_format == CFB_PIXEL_RG48) ? 6 : (out_format == CFB_PIXEL_B64A) ? 8 : 2;
-    *rowbytes = out_w * bpp; *dpitch = (out_w * bpp + 15) & ~15;
-    if ((out_format == CFB_PIXEL_YU64 || out_format == CFB_PIXEL_RG48 || rgb30) && (size_t)*dpitch * out_h > cd->frame_stride) {
+    *rowbytes = (out_format == CFB_PIXEL_V210) ? v210_row_bytes(out_w) : out_w * bpp;
+    *dpitch = (*rowbytes + 15) & ~15;
+    // a 4:2:2 codec's staging holds at least the three planar16 planes (4 W bytes per row), more than V210's 8 W / 3 + 16
+    if ((out_format == CFB_PIXEL_YU64 || out_format == CFB_PIXEL_RG48 || rgb30 || out_format == CFB_PIXEL_V210) &&
+        (size_t)*dpitch * out_h > cd->frame_stride) {
         set_error("packed output does not fit the codec's frame staging"); return CFB_ERROR_UNSUPPORTED;
     }
     if (out_format == CFB_PIXEL_PLANAR16) {

@@ -55,6 +55,11 @@ struct FwdParams {
 
 constexpr int kInvStrip = 120;    // band columns written per warp-row by the inverse kernels (30 lanes x 4)
 
+// output of the final 4:2:2 inverse level (k_inv_422)
+constexpr int kInv422Out8 = 0;    // packed 8-bit YUYV / UYVY
+constexpr int kInv422OutYU64 = 1; // packed 16-bit Y0 C1 Y1 C3
+constexpr int kInv422OutV210 = 2; // packed 10-bit V210, 6 pixels in 4 words
+
 struct InvGeom {
     int width;          // band width (coefficients)
     int height;         // band rows

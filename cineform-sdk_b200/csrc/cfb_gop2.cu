@@ -238,7 +238,7 @@ cfb_error cfb_gop2_inverse_host(cfb_codec *cd, const void *h_coded, const cfb_go
             aux.carry = cd->d_carry; aux.nstrips = cd->carry_strips; aux.maxh = p.ch[0].height; aux.pad = (cd->interlaced == 2);
             CFB_CUDA(launch_inv_fields(p, aux, false, ctx->stream));
         } else {
-            CFB_CUDA(launch_inv_422(p, false, ctx->stream));
+            CFB_CUDA(launch_inv_422(p, kInv422Out8, ctx->stream));
         }
         ctx->kernel_launches++;
         CFB_CUDA(cudaMemcpy2DAsync(dst[f], frame_pitch, dfr, L.frame_pitch, L.frame_pitch, (size_t)(L.frame_bytes / L.frame_pitch),

@@ -31,7 +31,8 @@ cudaError_t launch_fwd_rg48_all(const FwdParams &p, cudaStream_t stream);
 cudaError_t launch_fwd_byr4(const FwdParams &p, cudaStream_t stream);
 cudaError_t launch_fwd_rgb30(const FwdParams &p, cudaStream_t stream);
 cudaError_t launch_inv_plane(const InvParams &p, int descale, cudaStream_t stream);
-cudaError_t launch_inv_422(const InvParams &p, bool out16, cudaStream_t stream);
+// out: kInv422Out8 (YUYV / UYVY), kInv422OutYU64, kInv422OutV210 (cfb_common.cuh)
+cudaError_t launch_inv_422(const InvParams &p, int out, cudaStream_t stream);
 cudaError_t launch_inv_444_rg48(const InvParams &p, int out, cudaStream_t stream);
 cudaError_t launch_lowpass_422(const InvParams &p, cudaStream_t stream);
 cudaError_t launch_inv_fields(const InvParams &p, const FieldsAux &a, bool planar, cudaStream_t stream);

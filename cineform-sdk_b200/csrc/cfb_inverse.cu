@@ -447,12 +447,75 @@ __device__ __forceinline__ void emit_422(const InvParams &p, unsigned char *out,
     }
 }
 
-// OUT16 = false: packed 8-bit YUYV / UYVY.  OUT16 = true: packed 16-bit Y0 C1 Y1 C3 (YU64; C1 = channel 1, C3 = channel 2,
+// V210 output: component word of three 10-bit values at bits 0, 10, 20
+__device__ __forceinline__ unsigned v210_word(unsigned a, unsigned b, unsigned c) { return a | (b << 10) | (c << 20); }
+
+// One band row r of the final 4:2:2 level -> V210 rows 2r and 2r + 1 (decoder.c:26292 -> InvertHorizontalStrip16s.c:6490
+// InvertHorizontalYUVStrip16sToYUVOutput: the YU64 row rule, then convert.c:13526 ConvertPlanarYUVToV210 at precision 16).
+// A component is row16u >> 6 = min(max(t >> 1, 0), 1023): both of the 16-bit rule's limits (0xFFC0, 65535) become 1023.
+// Group of 6 pixels = 4 words: Cb0 Y0 Cr0 | Y1 Cb2 Y2 | Cr2 Y3 Cb4 | Y4 Cr4 Y5, Cb = channel 2 (the u arrays), Cr = channel 1.
+// A lane owns 8 pixels, so three writer lanes (phase 0, 1, 2 = (lane - 1) % 3) own 24 pixels = 4 groups = 64 bytes and a
+// strip (240 pixels) starts on a group boundary.  Phase 0 writes groups 0-1, phase 1 groups 2-3, phase 2 nothing; the part
+// of a group that belongs to the next lane arrives by one shuffle-down of six partial words, so every lane of the warp
+// must call this (`writer` gates the stores only).  `out` points at the lane's first byte of row 0 (its phase's groups).
+// right_edge (the lane holds the last 8 pixels of the row, widths are multiples of 16): the row ends inside a group, and
+// the reference's scalar tail (convert.c:13888-13965) fills the pixels past the edge with the component variables' last
+// values.  Phase 0 at the edge: W % 6 == 2, group 1 holds pixels W-2, W-1.  Phase 1 at the edge: W % 6 == 4, group 2
+// holds W-4 .. W-1, and no group 3 is written.  In that W % 6 == 4 group the reference's Cb field of word 2 reads one
+// element past the Cb row of its scratch strip (the next scratch row's first luma sample, or stale scratch on the
+// strip's last row); here it is defined as the last Cb of the row repeated.  Only ceil(W / 6) * 16 bytes per row are written.
+__device__ __forceinline__ void emit_v210(const InvParams &p, unsigned char *out, int phase, bool writer, bool right_edge, int r,
+                                          const int *ye, const int *yo, const int *ue, const int *uo, const int *ve, const int *vo)
+{
+    const InvGeom &gy = p.ch[0];
+    unsigned char *o = out + (long long)(2 * r) * gy.out_pitch;
+#pragma unroll
+    for (int rr = 0; rr < 2; rr++) {
+        const int *yy = rr ? yo : ye, *uu = rr ? uo : ue, *vv = rr ? vo : ve;
+        unsigned y[8], cb[4], cr[4];
+#pragma unroll
+        for (int i = 0; i < 8; i++) y[i] = row16u(yy[i], 0, 1023);
+#pragma unroll
+        for (int k = 0; k < 4; k++) { cb[k] = row16u(uu[k], 0, 1023); cr[k] = row16u(vv[k], 0, 1023); }
+        // what the previous lane needs from this one: phase 1 -> phase 0 (the rest of its group 1: pixels 0-3 here),
+        // phase 2 -> phase 1 (the rest of its group 2: pixels 0-1, and its whole group 3: pixels 2-7)
+        const bool p1 = (phase == 1);
+        unsigned s[6];
+        s[0] = p1 ? (cb[0] << 10) | (y[0] << 20) : cb[0] << 20;
+        s[1] = p1 ? v210_word(cr[0], y[1], cb[1]) : v210_word(y[0], cr[0], y[1]);
+        s[2] = p1 ? v210_word(y[2], cr[1], y[3]) : v210_word(cb[1], y[2], cr[1]);
+        s[3] = v210_word(y[3], cb[2], y[4]);
+        s[4] = v210_word(cr[2], y[5], cb[3]);
+        s[5] = v210_word(y[6], cr[3], y[7]);
+        unsigned n[6];
+#pragma unroll
+        for (int i = 0; i < 6; i++) n[i] = __shfl_down_sync(kFullMask, s[i], 1);
+        unsigned char *q = o + (rr ? gy.out_pitch : 0);
+        if (!writer) continue;
+        if (phase == 0) {
+            *reinterpret_cast<uint4 *>(q) = make_uint4(v210_word(cb[0], y[0], cr[0]), v210_word(y[1], cb[1], y[2]),
+                                                       v210_word(cr[1], y[3], cb[2]), v210_word(y[4], cr[2], y[5]));
+            *reinterpret_cast<uint4 *>(q + 16) =
+                right_edge ? make_uint4(v210_word(cb[3], y[6], cr[3]), v210_word(y[7], cb[3], y[6]), v210_word(cr[3], y[7], cb[3]),
+                                        v210_word(y[7], cr[3], y[6]))
+                           : make_uint4(v210_word(cb[3], y[6], cr[3]), y[7] | n[0], n[1], n[2]);
+        } else if (phase == 1) {
+            *reinterpret_cast<uint4 *>(q) =
+                make_uint4(v210_word(cb[2], y[4], cr[2]), v210_word(y[5], cb[3], y[6]),
+                           cr[3] | (y[7] << 10) | (right_edge ? cb[3] << 20 : n[0]), right_edge ? v210_word(y[7], cr[3], y[6]) : n[1]);
+            if (!right_edge) *reinterpret_cast<uint4 *>(q + 16) = make_uint4(n[2], n[3], n[4], n[5]);
+        }
+    }
+}
+
+// OUT = kInv422Out8: packed 8-bit YUYV / UYVY.  kInv422OutYU64: packed 16-bit Y0 C1 Y1 C3 (C1 = channel 1, C3 = channel 2,
 // as the YU64 encoder input assigns them), the reference's 16-bit row output (decoder.c:26351-26366 ->
 // TransformInverseSpatialUniversalThreadedToRow16u -> InvertHorizontalStrip16s.c:17462 / :16571) -- no dither, bit-exact.
-template <bool SMALLDQ, bool OUT16, int MINB>
+// kInv422OutV210: packed 10-bit V210 (emit_v210), bit-exact too.
+template <bool SMALLDQ, int OUT, int MINB>
 __global__ void __launch_bounds__(128, MINB) k_inv_422(const __grid_constant__ InvParams p)
 {
+    constexpr bool OUT16 = (OUT == kInv422OutYU64);
     const int lane = threadIdx.x;
     const int f = blockIdx.z;
     const InvGeom &gy = p.ch[0];
@@ -470,10 +533,16 @@ __global__ void __launch_bounds__(128, MINB) k_inv_422(const __grid_constant__ I
     const bool has_border = (strip == 0) || ((strip + 1) * kInvStrip + 4 >= gy.width);
     const unsigned ycol = (unsigned)(col0 * 2), ccol = (unsigned)col0;      // byte offsets (chroma: 2 columns of 2 bytes)
     const unsigned char *in = p.in_base[f];
-    unsigned char *out = p.out_base[f] + gy.out_off + (long long)col0 * (OUT16 ? 8 : 4);     // 2 (4) bytes per luma sample, 2 samples per column
+    // V210: lanes of phase (lane - 1) % 3 = (col0 % 12) / 4 write at 64 bytes per 12 band columns + 32 per phase
+    const int phase = (lane + 2) % 3;
+    unsigned char *out = p.out_base[f] + gy.out_off +
+                         (OUT == kInv422OutV210 ? (long long)(col0 / 12) * 64 + 32 * phase
+                                                : (long long)col0 * (OUT16 ? 8 : 4));     // 2 (4) bytes per luma sample, 2 samples per column
 
+    // every lane calls this (the V210 emitter shuffles); the 8- and 16-bit emitters run on the writer lanes only
     auto emit = [&](int r, const int *ye, const int *yo, const int *ue, const int *uo, const int *ve, const int *vo) {
-        emit_422<OUT16>(p, out, col0, r, ye, yo, ue, uo, ve, vo);
+        if constexpr (OUT == kInv422OutV210) emit_v210(p, out, phase, writer, right_border, r, ye, yo, ue, uo, ve, vo);
+        else if (writer) emit_422<OUT16>(p, out, col0, r, ye, yo, ue, uo, ve, vo);
     };
 
     if (blockIdx.y == gridDim.y - 1) {          // border warps: band rows 0 and H-1
@@ -483,7 +552,7 @@ __global__ void __launch_bounds__(128, MINB) k_inv_422(const __grid_constant__ I
         inv_border_row<4>(gy, in, bottom, H, ycol, active, has_border, left_border, right_border, ye, yo);
         inv_border_row<2>(gu, in, bottom, H, ccol, active, has_border, left_border, right_border, ue, uo);
         inv_border_row<2>(gv, in, bottom, H, ccol, active, has_border, left_border, right_border, ve, vo);
-        if (writer) emit(bottom ? H - 1 : 0, ye, yo, ue, uo, ve, vo);
+        emit(bottom ? H - 1 : 0, ye, yo, ue, uo, ve, vo);
         return;
     }
     const int y0 = max((int)(blockIdx.y * blockDim.y + threadIdx.y) * p.th, 1);
@@ -505,7 +574,7 @@ __global__ void __launch_bounds__(128, MINB) k_inv_422(const __grid_constant__ I
         inv_step<4, SMALLDQ>(sy, gy, in, r, y1, H, ycol, active, has_border, left_border, right_border, ye, yo);
         inv_step<2, SMALLDQ>(su, gu, in, r, y1, H, ccol, active, has_border, left_border, right_border, ue, uo);
         inv_step<2, SMALLDQ>(sv, gv, in, r, y1, H, ccol, active, has_border, left_border, right_border, ve, vo);
-        if (writer) emit(r, ye, yo, ue, uo, ve, vo);
+        emit(r, ye, yo, ue, uo, ve, vo);
     }
 }
 
@@ -886,12 +955,18 @@ static cudaError_t launch_inv_422_tma(const InvParams &p, const InvTmaMaps &tm, 
     }
 }
 
-cudaError_t launch_inv_422(const InvParams &p, bool out16, cudaStream_t stream)
+cudaError_t launch_inv_422(const InvParams &p, int out, cudaStream_t stream)
 {
     dim3 block(32, 4);
     dim3 grid(ceil_div_i(p.ch[0].width, kInvStrip), ceil_div_i(ceil_div_i(p.ch[0].height, p.th), (int)block.y) + 1, p.nframes);
     bool small = true;
     for (int c = 0; c < 3; c++) for (int b = 1; b < 4; b++) small = small && (p.ch[c].dq[b] >= 0 && p.ch[c].dq[b] <= 255);
+    if (out == kInv422OutV210) {        // register kernel only: the TMA variant lost its A/B (profiles/r02_ab_inv422.txt)
+        if (small) k_inv_422<true, kInv422OutV210, 4><<<grid, block, 0, stream>>>(p);
+        else k_inv_422<false, kInv422OutV210, 4><<<grid, block, 0, stream>>>(p);
+        return cudaGetLastError();
+    }
+    const bool out16 = (out == kInv422OutYU64);
     // The TMA path needs 16-byte aligned band starts and pitches (cfb_layout_compute guarantees both for pyramids it laid
     // out), whole 32-bit elements per band row, and LH / HL / HH of a channel equally spaced
     const int variant = inv422_variant();
@@ -919,9 +994,10 @@ cudaError_t launch_inv_422(const InvParams &p, bool out16, cudaStream_t stream)
         if (out16) return small ? launch_inv_422_tma<true, true>(p, tm, grid, block, variant, stream) : launch_inv_422_tma<false, true>(p, tm, grid, block, variant, stream);
         return small ? launch_inv_422_tma<true, false>(p, tm, grid, block, variant, stream) : launch_inv_422_tma<false, false>(p, tm, grid, block, variant, stream);
     }
-    if (out16) { if (small) k_inv_422<true, true, 3><<<grid, block, 0, stream>>>(p); else k_inv_422<false, true, 3><<<grid, block, 0, stream>>>(p); }
-    else if (variant == 5) { if (small) k_inv_422<true, false, 5><<<grid, block, 0, stream>>>(p); else k_inv_422<false, false, 5><<<grid, block, 0, stream>>>(p); }
-    else { if (small) k_inv_422<true, false, 4><<<grid, block, 0, stream>>>(p); else k_inv_422<false, false, 4><<<grid, block, 0, stream>>>(p); }
+    constexpr int O8 = kInv422Out8, O16 = kInv422OutYU64;
+    if (out16) { if (small) k_inv_422<true, O16, 3><<<grid, block, 0, stream>>>(p); else k_inv_422<false, O16, 3><<<grid, block, 0, stream>>>(p); }
+    else if (variant == 5) { if (small) k_inv_422<true, O8, 5><<<grid, block, 0, stream>>>(p); else k_inv_422<false, O8, 5><<<grid, block, 0, stream>>>(p); }
+    else { if (small) k_inv_422<true, O8, 4><<<grid, block, 0, stream>>>(p); else k_inv_422<false, O8, 4><<<grid, block, 0, stream>>>(p); }
     return cudaGetLastError();
 }
 

@@ -69,7 +69,7 @@ typedef enum cfb_pixel_format {
                              * (CFHD_PIXEL_FORMAT_YU64; frame.c:1556 ConvertYU64ToFrame16s); input only */
     CFB_PIXEL_V210 = 6,     /* 10-bit packed 4:2:2, components Cb Y Cr Y ... three per 32-bit word, rows padded to
                              * 128 bytes (CFHD_PIXEL_FORMAT_V210; encoder.c:2518 ConvertV210ToFrame16s: Cb -> channel 2,
-                             * Cr -> channel 1); input only */
+                             * Cr -> channel 1).  As an OUTPUT (4:2:2 codecs, full resolution, progressive): see cfb_inverse_device */
     /* 10-bit packed RGB, one 32-bit word per pixel -> 3 planes G, R, B at 12 bits like RG48 (encoder.c:3158-3176
      * TransformForwardSpatialRGB30, field layouts spatial.c:2118-2268); input only */
     CFB_PIXEL_RG30 = 7,     /* R bits 0-9, G 10-19, B 20-29 (CFHD_PIXEL_FORMAT_RG30)                       */
@@ -237,7 +237,17 @@ CFB_API cfb_error cfb_forward_host(cfb_codec *codec, int n, const void *const *h
  * InvertHorizontalStrip16s.c:14812: the 12-bit sample limited to [0, 4095], >> 2) from RGB 4:4:4 codecs (full resolution,
  * progressive).  The reference's LOWPASS BAND DECODE adds a per-output-format constant to LL3 (decoder.c:12270-12316: 6 for
  * the 10-bit RGB outputs, 8 for 8-bit RGB, 0 for RG48 / B64A ...): that belongs to the host's band decode, the caller
- * passes the bands as its decoder holds them. */
+ * passes the bands as its decoder holds them.
+ * CFB_PIXEL_V210 from 4:2:2 codecs, full resolution and progressive only (else CFB_ERROR_UNSUPPORTED; a 4:4:4 codec gives
+ * CFB_ERROR_BADFORMAT), bit-exact too: the reference renders it as YU64 rows (decoder.c:26292 ->
+ * InvertHorizontalStrip16s.c:6490, the same ...ToRow16u rule as YU64) converted by convert.c:13526 ConvertPlanarYUVToV210
+ * at precision 16, so every component is the YU64 sample >> 6 (both YU64 limits, 0xFFC0 and 65535, become 1023).  Words
+ * Cb0 Y0 Cr0 | Y1 Cb2 Y2 | Cr2 Y3 Cb4 | Y4 Cr4 Y5 per 6 pixels, bits 0 / 10 / 20, Cb = channel 2, Cr = channel 1.  When
+ * width % 6 != 0 the last group is completed as the reference's scalar tail does (convert.c:13888-13965: a component past
+ * the right edge repeats the value its variable there last held), except the Cb field of word 2 when width % 6 == 4, which the
+ * reference reads from outside the row (not reproducible); it is the row's last Cb here.  Exactly ceil(width / 6) * 16
+ * bytes are written per row; frame_pitch must be at least that and a multiple of 16 (the SDK's own pitch rounds the row
+ * to 128 bytes, SampleDecoder.cpp:367), the rest of the row is left untouched.  The LL3 constant of V210 is the YU64 one. */
 CFB_API cfb_error cfb_inverse_device(cfb_codec *codec, int n, void *const *d_pyramids, const cfb_quant *quant,
                                      int out_format, void *const *d_frames, int frame_pitch);
 CFB_API cfb_error cfb_inverse_host(cfb_codec *codec, int n, const void *const *h_coded, const cfb_quant *quant,

@@ -106,7 +106,15 @@ struct Plan {
     void *sparse = nullptr;         // pinned staging for the coded region in the sparse transfer format (allocated on first use)
     int curve_mode = -1;            // Bayer: encode curve the codec currently holds (-1 unknown, 0 none = curve applied, 1 = default log 90)
     void *frame = nullptr;          // pinned staging for a decoded frame at the ENCODED size (allocated on first use)
+    size_t frame_cap = 0;           // bytes of `frame` (outputs differ in size: 8-bit 4:2:2 .. B64A)
     bool ensure_coded() { return coded || cfb_host_alloc((size_t)layout.coded_bytes, &coded) == CFB_OK; }
+    bool ensure_frame(size_t bytes) {
+        if (frame && frame_cap >= bytes) return true;
+        if (frame) { cfb_host_free(frame); frame = nullptr; frame_cap = 0; }
+        if (cfb_host_alloc(bytes, &frame) != CFB_OK) { frame = nullptr; return false; }
+        frame_cap = bytes;
+        return true;
+    }
     bool ensure_sparse() { return sparse || cfb_host_alloc(cfb_sparse_max_bytes(&layout), &sparse) == CFB_OK; }
 };
 
@@ -596,14 +604,63 @@ void ComputeGroupTransformQuant(ENCODER *encoder, TRANSFORM *transform[], int nu
 }
 
 // ------------------------------------------------------------------------------------------------ decoder
+// The CFB_PIXEL_* output the decoder's DECODED_FORMAT_* maps to for this sample, -1 where the reference keeps the frame:
+//   4:2:2 samples, precision 10: 8-bit YUYV / UYVY, progressive or interlaced (field transform at level 1); YU64 and V210
+//     progressive only (decoder.c:26292 / :26351; the reference renders them from a field transform only through its
+//     active-metadata path, decoder.c:26413);
+//   RGB 4:4:4 samples, 3 channels, precision 12, progressive: RG48, B64A and the 10-bit words (decoder.c:26862-26907).
+// Everything else stays with the reference: RGB 4:4:4 -> YU64 / V210 (a colour conversion, TransformInverseRGB444ToYU64
+// at decoder.c:26874), 8-bit RGB, RG64, Bayer.
+static int gpu_output_format(const DECODER *d)
+{
+    const CODEC_STATE *cs = &d->codec;
+    if (cs->num_channels != 3) return -1;
+    const int f = d->frame.format;
+    if (cs->encoded_format == ENCODED_FORMAT_YUV_422 && cs->precision == 10) {
+        if (f == DECODED_FORMAT_YUYV) return CFB_PIXEL_YUYV;
+        if (f == DECODED_FORMAT_UYVY) return CFB_PIXEL_UYVY;
+        if (!cs->progressive) return -1;
+        if (f == DECODED_FORMAT_YU64) return CFB_PIXEL_YU64;
+        if (f == DECODED_FORMAT_V210) return CFB_PIXEL_V210;
+        return -1;
+    }
+    if (cs->encoded_format == ENCODED_FORMAT_RGB_444 && cs->precision == 12 && cs->progressive) {
+        switch (f) {
+        case DECODED_FORMAT_RG48: return CFB_PIXEL_RG48;
+        case DECODED_FORMAT_B64A: return CFB_PIXEL_B64A;
+        case DECODED_FORMAT_RG30: return CFB_PIXEL_RG30;
+        case DECODED_FORMAT_AB10: return CFB_PIXEL_AB10;
+        case DECODED_FORMAT_AR10: return CFB_PIXEL_AR10;
+        case DECODED_FORMAT_R210: return CFB_PIXEL_R210;
+        case DECODED_FORMAT_DPX0: return CFB_PIXEL_DPX0;
+        default: return -1;
+        }
+    }
+    return -1;
+}
+
+// bytes the inverse writes per row of `w` pixels in output format `fmt`
+static size_t output_row_bytes(int fmt, int w)
+{
+    switch (fmt) {
+    case CFB_PIXEL_YU64: case CFB_PIXEL_RG30: case CFB_PIXEL_AB10: case CFB_PIXEL_AR10: case CFB_PIXEL_R210: case CFB_PIXEL_DPX0:
+        return (size_t)w * 4;
+    case CFB_PIXEL_V210: return (size_t)(w + 5) / 6 * 16;
+    case CFB_PIXEL_RG48: return (size_t)w * 6;
+    case CFB_PIXEL_B64A: return (size_t)w * 8;
+    default: return (size_t)w * 2;
+    }
+}
+
 static bool decoder_on_gpu(DECODER *d)
 {
     if (!gpu_enabled() || !d) return false;
-    const CODEC_STATE *cs = &d->codec;
-    if (cs->num_channels != 3 || cs->precision != 10) return false;     // progressive or interlaced (field transform at level 1)
-    if (cs->encoded_format != ENCODED_FORMAT_YUV_422) return false;
+    const int out = gpu_output_format(d);
+    if (out < 0) return false;
+    // V210 packs 6 pixels per group, so a display window narrower than the coded row (4:2:2 rows are coded in multiples of
+    // 16 pixels) is not a prefix of it: decided here, before ReconstructWaveletBand skips the CPU levels
+    if (out == CFB_PIXEL_V210 && d->frame.width % 16) return false;
     if (d->frame.resolution != DECODED_RESOLUTION_FULL) return false;
-    if (d->frame.format != DECODED_FORMAT_YUYV && d->frame.format != DECODED_FORMAT_UYVY) return false;
     if (d->use_active_metadata_decoder || d->channel_blend_type) return false;
     if (d->uncompressed_chunk && d->uncompressed_size && d->sample_uncompressed) return false;
     for (int c = 0; c < 3; c++) if (!d->transform[c] || d->transform[c]->type != TRANSFORM_TYPE_SPATIAL) return false;
@@ -636,9 +693,13 @@ void ReconstructSampleFrameToBuffer(DECODER *decoder, int frame, uint8_t *output
         (decoder->flags & DECODER_FLAGS_RENDER)) {
         WaitForTransformThread(decoder);        // all entropy / bookkeeping jobs of this sample have finished
         IMAGE *y1 = decoder->transform[0]->wavelet[0];
-        // interlaced samples: the entropy decoder has already integrated the level-1 HL band (decoder.c:20822)
-        if (y1) plan = get_plan(y1->width * 2, y1->height * 2, decoder->frame.format == DECODED_FORMAT_YUYV ? CFB_PIXEL_YUYV : CFB_PIXEL_UYVY,
-                                decoder->codec.progressive ? CFB_PROGRESSIVE : CFB_INTERLACED_HL_INTEGRATED);
+        // the plan's source format only names the sample's family: 4:2:2 (the 8-bit outputs keep their own, as before) or
+        // RGB 4:4:4; the output format is chosen per call.  Interlaced samples: the entropy decoder has already
+        // integrated the level-1 HL band (decoder.c:20822)
+        const int out = gpu_output_format(decoder);
+        const int family = (out == CFB_PIXEL_YUYV || out == CFB_PIXEL_UYVY) ? out
+                         : (decoder->codec.encoded_format == ENCODED_FORMAT_YUV_422 ? CFB_PIXEL_YUYV : CFB_PIXEL_RG48);
+        if (y1) plan = get_plan(y1->width * 2, y1->height * 2, family, decoder->codec.progressive ? CFB_PROGRESSIVE : CFB_INTERLACED_HL_INTEGRATED);
     }
     bool ok = plan != nullptr;
     for (int c = 0; c < 3 && ok; c++)
@@ -685,26 +746,32 @@ void ReconstructSampleFrameToBuffer(DECODER *decoder, int frame, uint8_t *output
             }
         }
     const void *coded[1] = {sparse ? plan->sparse : plan->coded};
-    const int fmt = decoder->frame.format == DECODED_FORMAT_YUYV ? CFB_PIXEL_YUYV : CFB_PIXEL_UYVY;
+    const int fmt = gpu_output_format(decoder);
     // The pyramid has the ENCODED size (height rounded up to a multiple of 8, encoder.c:2232: 720x486 is coded as 488
     // rows) while the caller's buffer holds the DISPLAY size (decoder->frame): the reference writes info->height rows of
     // info->width pixels only.  When the two differ the frame is decoded into a staging buffer and the display window is
     // copied out, so nothing is ever written past the caller's last row.
     const int enc_w = plan->layout.band[0][0][0].width * 2, enc_h = plan->layout.band[0][0][0].height * 2;
     const int out_w = decoder->frame.width, out_h = decoder->frame.height;
-    if (out_w <= 0 || out_h <= 0 || out_w > enc_w || out_h > enc_h || pitch < out_w * 2) { g_inv_ref++; release_plans(); ref(decoder, frame, output, pitch); return; }
+    const size_t row_bytes = output_row_bytes(fmt, out_w);
+    // V210 packs 6 pixels per group, and its last group depends on the row width: a narrower display window is not a
+    // prefix of the coded row
+    const bool window_ok = out_w == enc_w || fmt != CFB_PIXEL_V210;
+    if (out_w <= 0 || out_h <= 0 || out_w > enc_w || out_h > enc_h || (size_t)pitch < row_bytes || !window_ok) {
+        g_inv_ref++; release_plans(); ref(decoder, frame, output, pitch); return;
+    }
     cfb_error err;
     if (out_w == enc_w && out_h == enc_h) {
         void *frames[1] = {output};
         err = sparse ? cfb_inverse_host_sparse(plan->codec, 1, coded, &q, fmt, frames, pitch) : cfb_inverse_host(plan->codec, 1, coded, &q, fmt, frames, pitch);
     } else {
-        if (!plan->frame && cfb_host_alloc((size_t)plan->layout.frame_bytes, &plan->frame) != CFB_OK) plan->frame = nullptr;
-        void *frames[1] = {plan->frame};
-        err = !plan->frame ? CFB_ERROR_OUTOFMEMORY : sparse ? cfb_inverse_host_sparse(plan->codec, 1, coded, &q, fmt, frames, plan->layout.frame_pitch)
-                                                           : cfb_inverse_host(plan->codec, 1, coded, &q, fmt, frames, plan->layout.frame_pitch);
+        const int fpitch = (int)((output_row_bytes(fmt, enc_w) + 15) & ~(size_t)15);
+        void *frames[1] = {plan->ensure_frame((size_t)fpitch * enc_h) ? plan->frame : nullptr};
+        err = !frames[0] ? CFB_ERROR_OUTOFMEMORY : sparse ? cfb_inverse_host_sparse(plan->codec, 1, coded, &q, fmt, frames, fpitch)
+                                                         : cfb_inverse_host(plan->codec, 1, coded, &q, fmt, frames, fpitch);
         if (err == CFB_OK)
             for (int r = 0; r < out_h; r++)
-                memcpy(output + (size_t)r * pitch, (const char *)plan->frame + (size_t)r * plan->layout.frame_pitch, (size_t)out_w * 2);
+                memcpy(output + (size_t)r * pitch, (const char *)plan->frame + (size_t)r * fpitch, row_bytes);
     }
     if (err != CFB_OK) {
         fprintf(stderr, "cfhd_gpu_shim: CUDA inverse failed: %s\n", cfb_last_error_string());

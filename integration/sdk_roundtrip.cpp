@@ -4,13 +4,16 @@
 // Linked twice by integration/Makefile: against libCFHDCodec.so (CUDA transform interposed) and against the plain
 // reference, so the same program times both and their outputs can be compared.
 //
-//   sdk_roundtrip <width> <height> <frames> [pool_threads [queue [interlaced [format]]]]
-// format: yuy2 (default; the only one that is also decoded), 2vuy, yu64, v210, rg48, rg30, r210, dpx0, ab10, ar10, byr4 --
-// the source formats whose level-1 kernels libcfhd_b200 has; V210 and BYR4 frames (which Example/qbist.cpp cannot draw)
-// are packed here from its YU64 / RG48 frames.
+//   sdk_roundtrip <width> <height> <frames> [pool_threads [queue [interlaced [format [decode]]]]]
+// format: yuy2 (default), 2vuy, yu64, v210, rg48, rg30, r210, dpx0, ab10, ar10, byr4 -- the source formats whose level-1
+// kernels libcfhd_b200 has; V210 and BYR4 frames (which Example/qbist.cpp cannot draw) are packed here from its YU64 /
+// RG48 frames.
+// decode: without it only yuy2 samples are decoded (to YUY2, with a dither-insensitive digest).  "same" decodes every
+// sample into its own source format; a format name (e.g. b64a for rg48 samples) decodes into that one.  The digest of the
+// decoded frames then covers every byte of every decoded frame (none of these outputs is dithered).
 // prints one JSON line: sync encode/decode ms, sample bytes, FNV-1a digests of the encoded samples (sync loop and pool;
 // from byte 512 on: the sample header carries the wall-clock time of the encode as metadata, bytes 155-180 at 640x96),
-// luma PSNR, digest of the decoded frames, pool fps.
+// luma PSNR (yuy2 decodes), digest of the decoded frames, pool fps.
 #include <math.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -47,15 +50,25 @@ int main(int argc, char **argv)
         {"ab10", CFHD_PIXEL_FORMAT_AB10, CFHD_PIXEL_FORMAT_AB10, CFHD_ENCODED_FORMAT_RGB_444, 4, 1},
         {"ar10", CFHD_PIXEL_FORMAT_AR10, CFHD_PIXEL_FORMAT_AR10, CFHD_ENCODED_FORMAT_RGB_444, 4, 1},
         {"byr4", CFHD_PIXEL_FORMAT_BYR4, CFHD_PIXEL_FORMAT_RG48, CFHD_ENCODED_FORMAT_BAYER, 2, 1},
+        {"b64a", CFHD_PIXEL_FORMAT_B64A, CFHD_PIXEL_FORMAT_B64A, CFHD_ENCODED_FORMAT_RGB_444, 8, 1},     // decode only
     };
-    const Fmt *F = nullptr;
+    const Fmt *F = nullptr, *D = nullptr;
     for (const Fmt &t : table) if (!strcmp(t.name, fname)) F = &t;
-    if (!F) { fprintf(stderr, "unknown format %s\n", fname); return 1; }
+    if (!F || F->fmt == CFHD_PIXEL_FORMAT_B64A) { fprintf(stderr, "unknown source format %s\n", fname); return 1; }
+    const char *dname = argc > 8 ? argv[8] : nullptr;
+    if (dname) {
+        for (const Fmt &t : table) if (!strcmp(t.name, strcmp(dname, "same") ? dname : fname)) D = &t;
+        if (!D) { fprintf(stderr, "unknown decode format %s\n", dname); return 1; }
+    }
     const bool is_yuy2 = F->fmt == CFHD_PIXEL_FORMAT_YUY2;
     const bool is_v210 = F->fmt == CFHD_PIXEL_FORMAT_V210, is_byr4 = F->fmt == CFHD_PIXEL_FORMAT_BYR4;
     CFHD_EncodingFlags eflags = interlaced ? CFHD_ENCODING_FLAGS_YUV_INTERLACED : CFHD_ENCODING_FLAGS_NONE;
     if (is_byr4) eflags = CFHD_ENCODING_FLAGS_CURVE_APPLIED;        // the mosaic already carries its curve
     const int pitch = is_v210 ? ((w + 47) / 48) * 128 : w * F->bytes_num / F->bytes_den;
+    // the decoded frame: the source layout unless a decode format was named (V210: the SDK's 128-byte row rounding)
+    const CFHD_PixelFormat dfmt = D ? D->fmt : F->fmt;
+    const int dpitch = !D ? pitch : D->fmt == CFHD_PIXEL_FORMAT_V210 ? ((w + 47) / 48) * 128 : w * D->bytes_num / D->bytes_den;
+    const bool decode = is_yuy2 || D;
     const CFHD_PixelFormat fmt = F->fmt;
     const CFHD_EncodedFormat encfmt = F->enc;
     std::vector<uint8_t *> frames;
@@ -100,9 +113,10 @@ int main(int argc, char **argv)
     if (e) { fprintf(stderr, "decoder open failed: %d\n", (int)e); return 1; }
     // 16 guard rows behind the decoded frame: a decoder that writes the ENCODED height (rounded up to a multiple of 8,
     // e.g. 488 rows for a 720x486 source) instead of the display height would trample them
-    const size_t guard_bytes = (size_t)pitch * 16;
-    uint8_t *out = (uint8_t *)aligned((size_t)pitch * h + guard_bytes);
-    memset(out + (size_t)pitch * h, 0xA5, guard_bytes);
+    const size_t guard_bytes = (size_t)dpitch * 16;
+    uint8_t *out = (uint8_t *)aligned((size_t)dpitch * h + guard_bytes);
+    memset(out + (size_t)dpitch * h, 0xA5, guard_bytes);
+    int decoded = 0;
     double enc_s = 0, dec_s = 0, mse_sum = 0;
     size_t bytes = 0;
     uint64_t hash = 1469598103934665603ull, sample_hash = 1469598103934665603ull, pool_hash = 1469598103934665603ull;
@@ -123,25 +137,31 @@ int main(int argc, char **argv)
             bytes += size;
             for (size_t k = 512; k < size; k++) { sample_hash ^= ((const uint8_t *)sample)[k]; sample_hash *= 1099511628211ull; }
         }
-        if (!is_yuy2) continue;     // the other sources are encode-only here (the shim's decode side covers 8-bit 4:2:2 output)
+        if (!decode) continue;      // without a decode format the other sources are encode-only here
         if (!prepared) {
             int aw, ah; CFHD_PixelFormat af;
-            e = CFHD_PrepareToDecode(dec, w, h, fmt, CFHD_DECODED_RESOLUTION_FULL, CFHD_DECODING_FLAGS_NONE, sample, size, &aw, &ah, &af);
+            e = CFHD_PrepareToDecode(dec, w, h, dfmt, CFHD_DECODED_RESOLUTION_FULL, CFHD_DECODING_FLAGS_NONE, sample, size, &aw, &ah, &af);
             if (e) { fprintf(stderr, "CFHD_PrepareToDecode failed: %d\n", (int)e); return 3; }
+            if (D && af != dfmt) { fprintf(stderr, "CFHD_PrepareToDecode chose another output format\n"); return 3; }
             prepared = true;
         }
         t0 = now_s();
-        e = CFHD_DecodeSample(dec, sample, size, out, pitch);
+        e = CFHD_DecodeSample(dec, sample, size, out, dpitch);
         if (i >= 0) dec_s += now_s() - t0;
         if (e) { fprintf(stderr, "CFHD_DecodeSample failed: %d\n", (int)e); return 4; }
         if (i < 0) continue;
+        decoded++;
+        if (D) {                    // exact digest of the whole decoded frame
+            for (size_t k = 0; k < (size_t)dpitch * h; k++) { hash ^= out[k]; hash *= 1099511628211ull; }
+            continue;
+        }
         double mse = 0;
         for (size_t k = 0; k < (size_t)pitch * h; k += 2) { const double d = (double)out[k] - (double)f[k]; mse += d * d; }
         mse_sum += mse / ((double)w * h);
         for (size_t k = 0; k < (size_t)pitch * h; k += 97) { hash ^= (uint64_t)(out[k] >> 1); hash *= 1099511628211ull; }     // dither-insensitive digest
     }
     bool guard_ok = true;
-    for (size_t k = 0; k < guard_bytes; k++) guard_ok = guard_ok && out[(size_t)pitch * h + k] == 0xA5;
+    for (size_t k = 0; k < guard_bytes; k++) guard_ok = guard_ok && out[(size_t)dpitch * h + k] == 0xA5;
     const double psnr = 10.0 * log10(255.0 * 255.0 / (mse_sum / nframes + 1e-12));
 
     // asynchronous encoder pool, exactly the TestCFHD -E call sequence (TestCFHD.cpp:783-1047)
@@ -180,10 +200,12 @@ int main(int argc, char **argv)
     }
     printf("{\"width\": %d, \"height\": %d, \"frames\": %d, \"enc_ms\": %.3f, \"dec_ms\": %.3f, \"sample_bytes\": %zu, "
            "\"sample_digest\": \"%016llx\", \"pool_sample_digest\": \"%016llx\", "
-           "\"luma_psnr_db\": %.3f, \"decoded_digest\": \"%016llx\", \"pool_threads\": %d, \"pool_fps\": %.1f, \"interlaced\": %d, \"guard_ok\": %d, \"format\": \"%s\"}\n",
+           "\"luma_psnr_db\": %.3f, \"decoded_digest\": \"%016llx\", \"pool_threads\": %d, \"pool_fps\": %.1f, \"interlaced\": %d, \"guard_ok\": %d, \"format\": \"%s\"",
            w, h, nframes, 1e3 * enc_s / nframes, 1e3 * dec_s / nframes, bytes / nframes, (unsigned long long)sample_hash, (unsigned long long)pool_hash,
            psnr, (unsigned long long)hash,
            pool_threads, pool_fps, interlaced ? 1 : 0, guard_ok ? 1 : 0, fname);
+    if (D) printf(", \"decode_format\": \"%s\", \"decoded_frames\": %d", D->name, decoded);
+    printf("}\n");
     CFHD_CloseEncoder(enc);
     CFHD_CloseDecoder(dec);
     return 0;
